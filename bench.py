@@ -6,7 +6,7 @@ A *step* is one pass of the hot path: GCNConv(F, F) forward + backward (out.back
 whole graph, graph structure cached (GCNConv(cached=True) semantics in both arms).
 edges/sec = E_input * layers / t (E_input counted before self-loop insertion, SURVEY.md 8(d)).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 N=1 workload: N=10M nodes, E=100M edges, F=256, fp32 (the north-star headline shape; inputs of
 10 GB >> 126 MB L2, so no explicit L2 flush is needed).  N>1: weak scaling -- every rank owns a
@@ -28,6 +28,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True           # the benchmark writes nothing into the source tree (it may be read-only)
 
 
 # --------------------------------------------------------------------------- helpers
@@ -164,6 +165,27 @@ def pass_bytes(E_prime: int, N: int, F: int, s: int = 4, b_idx: int = 4, b_w: in
     return E_prime * (F * s + b_idx + b_w) + N * F * s + (N + 1) * b_idx
 
 
+DUMP_BYTES = 60_000_000                  # --dump-outputs: all arrays together stay below 64 MB
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """`--dump-outputs`: the results the timed path returned in its last step, as <out_dir>/<name>.npy in float32 (float64
+    stays float64), so that two builds can be compared output for output on the same seeded inputs.  An array larger than
+    its share of DUMP_BYTES is cut to a fixed, seeded sample of its rows: arrays with the same number of rows keep the
+    same rows, in ascending order."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach()
+        t = t if t.dtype == torch.float64 else t.float()
+        if t.numel() * t.element_size() > budget:
+            keep = budget // (t[0].numel() * t.element_size())
+            rows = torch.randperm(t.size(0), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t[rows.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 # --------------------------------------------------------------------------- the CPU reference arm
 def workload_config(args, world: int) -> dict:
     """The workload both arms are quoted on (identical dict in the b200 and the reference line)."""
@@ -174,8 +196,8 @@ def workload_config(args, world: int) -> dict:
 
 
 def _import_reference():
-    """The UNMODIFIED reference package installed by baseline/install_ref.sh (git-ignored, travels with gpurun)."""
-    ref = os.path.join(ROOT, "baseline", "_ref")
+    """The UNMODIFIED reference package, where build() installed it (oracle/install_ref.sh; git-ignored)."""
+    ref = os.path.join(ROOT, "oracle", "_ref")
     if os.path.isdir(os.path.join(ref, "torch_geometric")):
         if ref not in sys.path:
             sys.path.insert(0, ref)
@@ -194,7 +216,7 @@ def _cpu_threads() -> int:
 
 def _reference_step_fn(args):
     """(step, kind, how): one GCNConv(F, F, cached=True) forward+backward on the bounded CPU sample -- through the
-    reference's own GCNConv when baseline/_ref is installed, else through the restated ATen call sequence."""
+    reference's own GCNConv when oracle/_ref is installed, else through the restated ATen call sequence."""
     N, E, F = args.cpu_nodes, args.cpu_edges, args.feat
     torch.manual_seed(0)
     ei = synth_graph(N, E, 1, "cpu")
@@ -208,7 +230,7 @@ def _reference_step_fn(args):
             x.grad = None
             conv.zero_grad(set_to_none=True)
             conv(x, ei).backward(gout)
-        return step, "reference", f"torch_geometric {tg.__version__} GCNConv (baseline/_ref, unmodified), default [2,E] tensor path"
+        return step, "reference", f"torch_geometric {tg.__version__} GCNConv (oracle/_ref, unmodified), default [2,E] tensor path"
     from oracle import ref_aten
     weight = torch.nn.Parameter(torch.randn(F, F) / F ** 0.5)
     bias = torch.nn.Parameter(torch.zeros(F))
@@ -217,7 +239,7 @@ def _reference_step_fn(args):
     def step():
         x.grad = weight.grad = bias.grad = None
         ref_aten.gcn_conv_forward(x, ei2, w2, weight, bias).backward(gout)
-    return step, "port", "oracle/ref_aten.py (the reference's ATen call sequence; baseline/_ref not installed)"
+    return step, "port", "oracle/ref_aten.py (the reference's ATen call sequence; oracle/_ref not installed)"
 
 
 def run_reference(args):
@@ -447,8 +469,10 @@ def run_b200(args):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     sync_all()
     ev0.record()
+    out = None
     for _ in range(args.steps):
-        step()
+        out = None                          # released before the next step allocates, as if it were not kept
+        out = step()
     ev1.record()
     sync_all()
     ms = ev0.elapsed_time(ev1)
@@ -462,6 +486,10 @@ def run_b200(args):
         ms = float(t.item())
     ms_per_step = ms / args.steps
     value = world * E / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"out": out, "grad_x": x.grad, "grad_weight": conv.lin.weight.grad,
+                                         "grad_bias": conv.bias.grad})
+    del out
 
     # ---- end to end through the public API with HOST buffers (N=1 path; per rank for N>1)
     e2e = None
@@ -646,7 +674,14 @@ def main():
     ap.add_argument("--parity-rows", type=int, default=4096)
     ap.add_argument("--traffic-bytes", type=float, default=None,
                     help="dram bytes per launch of the dominant kernel from the committed ncu capture (profiles/)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (output, gradients of the input and "
+                         "of the parameters) as DIR/<name>.npy; at N > 1 rank 0's rows; not with --impl reference")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs records the B200 path; the reference arm has nothing to dump")
     if args.impl == "reference":
         run_reference(args)
     else:

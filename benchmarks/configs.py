@@ -148,8 +148,10 @@ def run_config(args, B):
     l0 = ops.LAUNCHES.count
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
+    out = None
     for _ in range(args.steps):
-        step()
+        out = None                          # released before the next step allocates, as if it were not kept
+        out = step()
     ev1.record()
     torch.cuda.synchronize()
     ms = ev0.elapsed_time(ev1)
@@ -159,6 +161,10 @@ def run_config(args, B):
     clocks = sampler.stop()
     ms_per_step = ms / args.steps
     value = E * layers / (ms_per_step * 1e-3)
+    if args.dump_outputs:
+        B.dump_outputs(args.dump_outputs, {"out": out, "grad_x": x.grad,
+                                           **{f"grad_param{i}": p.grad for i, p in enumerate(params)}})
+    del out
 
     # ---- roofline of the dominant kernel (forward launches; the backward sweeps are listed per op in `kernels`)
     agg = kern.get(dom_op, {"ms_total": 0.0, "calls": 0, "ms_each": []})

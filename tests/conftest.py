@@ -12,7 +12,7 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
 def pytest_configure(config):
-    config.addinivalue_line("markers", "gpu: needs a real B200 (run with -m gpu under gpurun)")
+    config.addinivalue_line("markers", "gpu: needs a real B200 (select with -m gpu)")
 
 
 @pytest.fixture(scope="session", autouse=True)
@@ -49,12 +49,10 @@ def assert_close(a, b, rtol=1e-5, atol=1e-6, msg=""):
 
 
 def reference_path():
-    """Where the UNMODIFIED reference package can be imported from: baseline/_ref (installed by
-    baseline/install_ref.sh; travels to the GPU box with the snapshot) or /root/reference (build container only)."""
-    for cand in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isdir(os.path.join(cand, "torch_geometric")):
-            return cand
-    return None
+    """Where the UNMODIFIED reference package can be imported from: oracle/_ref, installed by build() from the
+    reference checkout (oracle/install_ref.sh)."""
+    cand = os.path.join(ROOT, "oracle", "_ref")
+    return cand if os.path.isdir(os.path.join(cand, "torch_geometric")) else None
 
 
 @pytest.fixture
@@ -62,7 +60,7 @@ def tg():
     """The reference package (`import torch_geometric`); the test is skipped where it is not installed."""
     path = reference_path()
     if path is None:
-        pytest.skip("the reference package is not installed (baseline/install_ref.sh)")
+        pytest.skip("the reference package is not installed (oracle/install_ref.sh)")
     if path not in sys.path:
         sys.path.insert(0, path)
     import torch_geometric

@@ -55,24 +55,37 @@ def test_state_dict_layout_matches_reference_layers():
     assert sd["weight"].shape == (3, 8, 16) and sd["root"].shape == (8, 16) and sd["bias"].shape == (16, )
 
 
-def test_state_dict_names_and_shapes_equal_the_reference_layers(tg):
+def _mlp():
+    return torch.nn.Sequential(torch.nn.Linear(8, 16), torch.nn.ReLU(), torch.nn.Linear(16, 16))
+
+
+# (layer, args, kwargs); tests/golden/state_dicts.npz holds the reference layer's state_dict for each case
+# (tests/golden/make_golden_api.py), so a change here needs that file regenerated
+STATE_DICT_CASES = [
+    ("GCNConv", (8, 16), {}), ("SAGEConv", (8, 16), {}), ("SAGEConv", (8, 16), {"project": True}),
+    ("GATConv", (8, 4), {"heads": 3}), ("GATConv", (8, 4), {"heads": 2, "concat": False, "residual": True}),
+    ("RGCNConv", (8, 16, 3), {}), ("GINConv", (_mlp(), ), {"train_eps": True}), ("GINConv", (_mlp(), ), {}),
+    ("GATConv", (8, 4), {"heads": 2, "edge_dim": 3}), ("GATConv", ((8, 6), 4), {"heads": 2}),
+    ("GATv2Conv", (8, 4), {"heads": 3, "edge_dim": 5}),
+    ("GATv2Conv", (8, 4), {"heads": 2, "share_weights": True, "residual": True, "concat": False}),
+    ("TransformerConv", (8, 4), {"heads": 3, "edge_dim": 5, "beta": True}),
+    ("TransformerConv", (8, 4), {"heads": 2, "concat": False, "bias": False}),
+    ("GraphConv", (8, 16), {}), ("RGCNConv", (8, 16, 3), {"num_bases": 2}), ("RGCNConv", (8, 16, 3), {"num_blocks": 4}),
+    ("FastRGCNConv", (8, 16, 3), {}), ("HeteroLinear", (8, 16, 3), {}), ("HeteroLinear", (8, 16, 3), {"bias": False})]
+
+
+def test_state_dict_names_and_shapes_equal_the_reference_layers(golden):
     """Checkpoints are interchangeable: same keys AND shapes as the reference's layers, option by option (GIN's eps is [1],
     `edge_dim` adds `lin_edge` / `att_edge`, `share_weights` registers one module under two names, ...)."""
     import pytorch_geometric_b200.nn as ours
-    mlp = lambda: torch.nn.Sequential(torch.nn.Linear(8, 16), torch.nn.ReLU(), torch.nn.Linear(16, 16))   # noqa: E731
-    cases = [("GCNConv", (8, 16), {}), ("SAGEConv", (8, 16), {}), ("SAGEConv", (8, 16), {"project": True}),
-             ("GATConv", (8, 4), {"heads": 3}), ("GATConv", (8, 4), {"heads": 2, "concat": False, "residual": True}),
-             ("RGCNConv", (8, 16, 3), {}), ("GINConv", (mlp(), ), {"train_eps": True}), ("GINConv", (mlp(), ), {}),
-             ("GATConv", (8, 4), {"heads": 2, "edge_dim": 3}), ("GATConv", ((8, 6), 4), {"heads": 2}),
-             ("GATv2Conv", (8, 4), {"heads": 3, "edge_dim": 5}),
-             ("GATv2Conv", (8, 4), {"heads": 2, "share_weights": True, "residual": True, "concat": False}),
-             ("TransformerConv", (8, 4), {"heads": 3, "edge_dim": 5, "beta": True}),
-             ("TransformerConv", (8, 4), {"heads": 2, "concat": False, "bias": False}),
-             ("GraphConv", (8, 16), {}), ("RGCNConv", (8, 16, 3), {"num_bases": 2}), ("RGCNConv", (8, 16, 3), {"num_blocks": 4}),
-             ("FastRGCNConv", (8, 16, 3), {}), ("HeteroLinear", (8, 16, 3), {}), ("HeteroLinear", (8, 16, 3), {"bias": False})]
-    for name, args, kw in cases:
+    ref = {}
+    for key, v in golden("state_dicts").items():
+        case, name = key.split("|", 1)
+        ref.setdefault(int(case), {})[name] = torch.from_numpy(v)
+    assert sorted(ref) == list(range(len(STATE_DICT_CASES)))
+    for i, (name, args, kw) in enumerate(STATE_DICT_CASES):
         a = getattr(ours, name)(*args, **kw).state_dict()
-        b = getattr(tg.nn, name)(*args, **kw).state_dict()
+        b = ref[i]
         assert {k: tuple(v.shape) for k, v in a.items()} == {k: tuple(v.shape) for k, v in b.items()}, (name, kw)
         getattr(ours, name)(*args, **kw).load_state_dict(b)          # a reference checkpoint loads
 

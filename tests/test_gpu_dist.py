@@ -159,23 +159,23 @@ def test_sharded_gcn_conv_single_rank_equals_unsharded():
     _launch(1)
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 def test_sharded_gcn_conv_two_ranks_nccl_equals_unsharded():
     _launch(2)
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 def test_peer_memory_gcn_conv_two_ranks_equals_unsharded():
     """Halo rows gathered over NVLink peer memory inside the kernel (dist_p2p.py)."""
     _launch(2, "p2p")
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 def test_peer_memory_two_stacked_layers_share_one_shard_forward_only():
     _launch(2, "p2p_stack")
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 def test_peer_memory_rgcn_conv_two_ranks_equals_unsharded():
     """BASELINE config 5 (RGCNConv, 2 x B200): the reduce-agnostic peer-sharded aggregate under the relational layer."""
     _launch(2, "p2p_rgcn")

@@ -1,4 +1,4 @@
-"""GPU tests of the reference-side binding: the UNMODIFIED reference package (baseline/_ref, fixture `tg`) running on
+"""GPU tests of the reference-side binding: the UNMODIFIED reference package (oracle/_ref, fixture `tg`) running on
 cuda with `pytorch_geometric_b200.plugin.install()`, compared with the same reference objects on the CPU (no plug-in
 involved there: CPU tensors fall through).
 
@@ -265,7 +265,7 @@ def test_subclass_layer_with_a_hook_falls_through_to_the_reference_propagate(tg,
 
 
 # ------------------------------------------------------------------------------------------------ (out, arg) operators
-def test_scatter_max_and_spmm_max_return_the_arg(tg, plugin):
+def test_scatter_max_and_spmm_max_return_the_arg():
     from pytorch_geometric_b200.plugin import shims
     ts = shims.torch_scatter_module()
     assert shims.register_torch_sparse_ops()
@@ -301,25 +301,18 @@ def test_scatter_max_and_spmm_max_return_the_arg(tg, plugin):
     del order
 
 
-def test_index_bookkeeping_mirrors_match_the_reference(tg):
+def test_index_bookkeeping_mirrors_match_the_reference(golden):
     """scatter_argmax / group_argsort / group_cat (utils/_scatter.py:145-300) of the standalone mirror vs the reference's own
-    functions on the CPU (tie-free values: the reference leaves ties to the order of a duplicate-index assignment)."""
+    functions run on the CPU (tests/golden/index_bookkeeping.npz; tie-free values: the reference leaves ties to the order
+    of a duplicate-index assignment)."""
     from pytorch_geometric_b200 import utils as U
-    g = torch.Generator().manual_seed(12)
-    N, E = 70, 900
-    index = torch.randint(0, N - 5, (E, ), generator=g)
-    src = torch.randperm(E, generator=g).float() * 0.37 - 100.0
-    from torch_geometric.utils._scatter import scatter_argmax as ref_argmax        # (not re-exported by utils/__init__)
-    want = ref_argmax(src, index, dim_size=N)
-    got = U.scatter_argmax(src.to(DEV), index.to(DEV), dim_size=N)
-    assert torch.equal(got.cpu(), want)
-    assert torch.equal(U.scatter_argmax(src.to(DEV), index.to(DEV)).cpu(), ref_argmax(src, index))
-    for kw in ({}, {"descending": True}, {"return_consecutive": True}, {"stable": True, "num_groups": N}):
-        want = tg.utils.group_argsort(src, index, **kw)
-        got = U.group_argsort(src.to(DEV), index.to(DEV), **kw)
-        assert torch.equal(got.cpu(), want), kw
-    x1, x2 = torch.randn(40, 3, generator=g), torch.randn(25, 3, generator=g)
-    i1, i2 = torch.sort(torch.randint(0, 9, (40, ), generator=g))[0], torch.sort(torch.randint(0, 9, (25, ), generator=g))[0]
-    want, wi = tg.utils.group_cat([x1, x2], [i1, i2], return_index=True)
-    got, gi = U.group_cat([x1.to(DEV), x2.to(DEV)], [i1.to(DEV), i2.to(DEV)], return_index=True)
-    assert torch.equal(got.cpu(), want) and torch.equal(gi.cpu(), wi)
+    ref = {k: torch.from_numpy(v) for k, v in golden("index_bookkeeping").items()}
+    N, src, index = int(ref["N"]), ref["src"].to(DEV), ref["index"].to(DEV)
+    assert torch.equal(U.scatter_argmax(src, index, dim_size=N).cpu(), ref["argmax_dim_size"])
+    assert torch.equal(U.scatter_argmax(src, index).cpu(), ref["argmax"])
+    for tag, kw in (("plain", {}), ("descending", {"descending": True}), ("consecutive", {"return_consecutive": True}),
+                    ("stable", {"stable": True, "num_groups": N})):
+        got = U.group_argsort(src, index, **kw)
+        assert torch.equal(got.cpu(), ref[f"group_argsort_{tag}"]), kw
+    got, gi = U.group_cat([ref["x1"].to(DEV), ref["x2"].to(DEV)], [ref["i1"].to(DEV), ref["i2"].to(DEV)], return_index=True)
+    assert torch.equal(got.cpu(), ref["group_cat"]) and torch.equal(gi.cpu(), ref["group_cat_index"])
